@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the hot path (BASELINE.json metric: scored triples/pairs per second at d=100).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[1]): TransE, d=100, |E|=100k, |R|=500, batches of 1024 positives
 with 10 corrupted negatives each; region: forward + margin loss + backward (row gradients).
@@ -145,6 +145,31 @@ def make_indices(torch, gen, n_batches, n_ent=N_ENT, n_rel=N_REL, k_neg=K_NEG):
     return [x.contiguous() for x in (ph, pt, pr, cfmt)]
 
 
+DUMP_GRAD_SLOTS = 32_768           # gradient rows kept per table: 2 x 32768 x 100 floats = 26 MB
+
+
+def dump_outputs(out_dir, torch, last, model):
+    """What the last launch of the timed region returned to its caller -- per-batch losses, positive and negative
+    scores -- and the sparse gradients it left in .grad, as DIR/<name>.npy.  Each gradient is a COO tensor with one
+    row per gathered slot (3.1M entity slots at the default shape); a fixed, seeded sample of slots is written: the
+    slot positions, the table row each one updates and its gradient row."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    loss, pos, neg = last
+    arrays = {"loss_per_batch": loss, "pos_scores": pos, "neg_scores": neg}
+    for name in ("ent", "rel"):
+        g = getattr(model, name + "_embeddings").weight.grad
+        rows, vals = g._indices()[0], g._values()
+        pick = torch.randperm(rows.numel(), generator=torch.Generator().manual_seed(2024))[:DUMP_GRAD_SLOTS]
+        pick = pick.sort().values
+        arrays[name + "_grad_slots"] = pick.double()
+        arrays[name + "_grad_rows"] = rows[pick.to(rows.device)].double()
+        arrays[name + "_grad_values"] = vals[pick.to(vals.device)]
+    for name, t in arrays.items():
+        a = t.detach().cpu().numpy()
+        np.save(os.path.join(out_dir, name + ".npy"), a if a.dtype == np.float64 else a.astype(np.float32))
+
+
 # =============================================================================================================
 # reference arm
 # =============================================================================================================
@@ -237,8 +262,7 @@ def run_ours(args):
     def launch_device(s):
         ix = dev_sets[s % n_sets]
         model.zero_grad(set_to_none=True)
-        loss, _, _ = model.loss_step_corrupt(tuple(ix[:3]), ix[3], margin=1.0, batch_pos=BATCH)
-        return loss
+        return model.loss_step_corrupt(tuple(ix[:3]), ix[3], margin=1.0, batch_pos=BATCH)
 
     # ---- device-resident timing: K steps of `lps` launches ---------------------------------------------
     sampler = ClockSampler(local)
@@ -254,10 +278,12 @@ def run_ours(args):
     step_evs[0].record()
     for k in range(args.steps):
         for s in range(lps):
-            launch_device(k * lps + s)
+            last = launch_device(k * lps + s)
         step_evs[k + 1].record()
     t1.record()
     barrier()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, torch, last, model)
     total_ms = max_over_ranks(t0.elapsed_time(t1))
     step_ms = sorted(step_evs[k].elapsed_time(step_evs[k + 1]) for k in range(args.steps))
     launches = model.kernel_launches - launches0
@@ -638,6 +664,9 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-regions", action="store_true")
     ap.add_argument("--headline-only", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed launch computed (losses, scores, a seeded sample of the gradient rows) "
+                         "as DIR/<name>.npy")
     args = ap.parse_args()
     if args.impl == "reference":
         run_reference(args)

@@ -14,10 +14,9 @@ vectors for this path (SURVEY.md section 4), so the oracle is pinned against
 vectors produced by importing the unmodified reference classes in the build
 container: ``tests/golden/make_golden.py`` writes them, ``tests/golden/*.npz``
 holds them, ``tests/test_oracle_golden.py`` checks this file against them.
-It is also checked LIVE against the reference itself: ``tests/test_oracle_live_reference.py``
-runs the unmodified classes of ``baseline/_ref`` (a patched copy of the checkout made by
-``baseline/make_ref.py``) on the CPU at the BASELINE row widths (d = 100, 128) and compares
-every function below with the reference's forward / autograd / evaluate* / ranking output.
+It is also checked at the BASELINE row widths (d = 100, 128): ``tests/golden/make_golden_live.py`` records
+what the unmodified classes return, ``tests/test_oracle_live_reference.py`` compares every function below
+with that forward / autograd / evaluate* / ranking output.
 
 Conventions
 -----------

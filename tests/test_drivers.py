@@ -1,258 +1,37 @@
-"""The reference's unmodified drivers, alone and with the CUDA modules swapped in.
+"""The drop-in constructors start from the reference's tables.
 
 north_star: "nn.Modules with the same constructors and forward() signatures as the reference
-classes so the three run_*.py entry points and -model_type dispatch call them unchanged".
-These tests execute exactly that: ``baseline/_ref/run_{knowledge_representation,
-item_recommendation,knowledgable_recommendation}.py`` (base.py:128-175 dispatch ->
-knowledge_representation.py:107-219 / item_recommendation.py:77-194 /
-knowledgable_recommendation.py:192-408) on a synthetic dataset, once on the host cores with
-the reference's own model classes and once through ``python -m kgrec_b200.dropin`` on the GPU,
-same flags and seed.  The model tables start bit-identical (same generator consumption as the
-reference constructors), the host-side sampling is the reference's own code under the same
-``random.seed``, so the two runs see the same batches; what differs is fp32 re-association in
-the kernels.  Compared: every logged training-loss average and every logged evaluation metric,
-and the two checkpoints evaluated by the OTHER implementation (``-eval_only_mode``).
+classes so the three run_*.py entry points and -model_type dispatch call them unchanged".  With the
+same torch seed the package's model classes draw bit-identical initial tables (same generator
+consumption as the reference constructors, transE.py:31-46 ...) and leave the generator in the same
+state, so a driver that seeds torch sees the same model and the same batches afterwards.  The
+reference's tables and the draw after them are stored in ``tests/golden/dropin_init.npz``
+(recorded by ``tests/golden/make_golden_live.py``).
 """
-import os
-
 import numpy as np
-import pytest
 import torch
 
-import driver_harness as H
-
-needs_ref = pytest.mark.skipif(not H.reference_available(),
-                               reason="baseline/_ref not built (python baseline/make_ref.py needs the reference checkout)")
-
-COMMON = ["-dataset", "ml1m", "-embedding_size", "32", "-batch_size", "256", "-seed", "3", "-num_processes", "2",
-          "-optimizer_type", "Adagrad", "-learning_rate", "0.05", "-topn", "10"]
-
-
-@pytest.fixture(scope="module")
-def dataset(tmp_path_factory):
-    root = tmp_path_factory.mktemp("kgrec_data")
-    info = H.make_dataset(str(root), users=300, items=1200, ratings=20000, entities=600, relations=8, triples=30000)
-    info["root"] = str(root) + os.sep
-    return info
+_IMAP = {i: i for i in range(70)}
+_NMAP = {i: ((i * 7) % 40 if i % 3 else -1, i) for i in range(70)}
+DROPIN_INIT_CASES = [
+    ("transE", (False, 16, 50, 7)), ("transH", (True, 16, 50, 7)), ("transR", (False, 8, 50, 7)),
+    ("transUP", (False, 16, 50, 70, 5, True)), ("jTransUP", (False, 16, 50, 70, 40, 5, _IMAP, _NMAP, False, False)),
+]
 
 
-def _flags(dataset, *extra):
-    return COMMON + ["-data_path", dataset["root"]] + list(extra)
-
-
-# ---------------------------------------------------------------------------------------------
-# CPU: the reference copy itself runs (BASELINE.json configs[0]: bprmf plumbing), and the drop-in
-# constructors start from the same tables as the reference's
-# ---------------------------------------------------------------------------------------------
-@needs_ref
-def test_reference_bprmf_plumbing_on_cpu(dataset, tmp_path):
-    """configs[0]: `run_item_recommendation.py -model_type bprmf` on the host, end to end
-    (flags -> loaders -> trainer -> train loop -> fork-per-batch evaluation -> checkpoint)."""
-    log, ckpt, _ = H.run_driver("rec", _flags(dataset, "-model_type", "bprmf", "-rec_test_files", "valid.dat:test.dat",
-                                              "-training_steps", "120", "-eval_interval_steps", "60"),
-                                str(tmp_path), "bprmf_cpu", cpu=True)
-    assert len(log["rec"]) == 4 and len(log["train_loss"]) == 2          # 2 eval rounds x 2 files
-    assert all(0.0 <= v <= 1.0 for row in log["rec"] for v in row)
-    assert np.isfinite(log["train_loss"][1][0]) and log["train_loss"][1][0] > 0
-    assert os.path.exists(ckpt)
-
-
-@needs_ref
-def test_dropin_constructors_start_from_the_reference_tables():
+def test_dropin_constructors_start_from_the_reference_tables(golden):
     """Same torch seed -> bit-identical initial tables and generator state (transE.py:31-46 ...)."""
-    import sys
-    import warnings
-    for p in reversed(H.make_ref.env_paths()):
-        sys.path.insert(0, p)
-    import gflags  # noqa: F401  (the shim; restores numpy.asfarray)
-    warnings.filterwarnings("ignore")
-    from jTransUP.models import transE as rE, transH as rH, transR as rR, transUP as rU, jTransUP as rJ
     import kgrec_b200 as K
-    imap = {i: i for i in range(70)}
-    nmap = {i: ((i * 7) % 40 if i % 3 else -1, i) for i in range(70)}
-    cases = [(rE.TransEModel, K.TransEModel, (False, 16, 50, 7)), (rH.TransHModel, K.TransHModel, (True, 16, 50, 7)),
-             (rR.TransRModel, K.TransRModel, (False, 8, 50, 7)), (rU.TransUPModel, K.TransUPModel, (False, 16, 50, 70, 5, True)),
-             (rJ.jTransUPModel, K.jTransUPModel, (False, 16, 50, 70, 40, 5, imap, nmap, False, False))]
-    for ref_cls, our_cls, args in cases:
+    g = golden("dropin_init")
+    classes = {"transE": K.TransEModel, "transH": K.TransHModel, "transR": K.TransRModel, "transUP": K.TransUPModel,
+               "jTransUP": K.jTransUPModel}
+    for name, args in DROPIN_INIT_CASES:
         torch.manual_seed(11)
-        a = ref_cls(*args)
-        ra = torch.rand(3)
-        torch.manual_seed(11)
-        b = our_cls(*args)
+        b = classes[name](*args)
         rb = torch.rand(3)
-        sa, sb = a.state_dict(), b.state_dict()
-        assert set(sa) == set(sb)
-        for k in sa:
-            assert torch.equal(sa[k].cpu(), sb[k].cpu()), (ref_cls.__name__, k)
-        assert torch.equal(ra, rb)
-
-
-# ---------------------------------------------------------------------------------------------
-# GPU: unmodified drivers through the drop-in vs the reference alone
-# ---------------------------------------------------------------------------------------------
-def _close(a, b, rel, abs_):
-    return abs(a - b) <= abs_ + rel * max(abs(a), abs(b))
-
-
-def _compare_logs(ref, new, keys, loss_rel=2e-3, frac_abs=0.004, rank_rel=0.01):
-    for k in keys:
-        assert len(ref[k]) == len(new[k]) and len(ref[k]) > 0, (k, ref[k], new[k])
-        for row_r, row_n in zip(ref[k], new[k]):
-            for j, (x, y) in enumerate(zip(row_r, row_n)):
-                if k in ("train_loss", "joint_loss"):
-                    ok = _close(x, y, loss_rel, 1e-4)
-                elif k.startswith("kg") and j == 1:          # mean rank
-                    ok = _close(x, y, rank_rel, 0.5)
-                else:                                        # hit / f1 / p / r / ndcg in [0, 1]
-                    ok = _close(x, y, 0.0, frac_abs)
-                assert ok, "%s differs: reference %s vs drop-in %s" % (k, row_r, row_n)
-
-
-def _both(kind, dataset, tmp_path, name, flags, **tol):
-    log_dir = str(tmp_path)
-    ref, ref_ckpt, _ = H.run_driver(kind, flags, log_dir, name + "_ref", cpu=True)
-    new, new_ckpt, _ = H.run_driver(kind, flags, log_dir, name + "_b200", dropin=True)
-    return ref, new, ref_ckpt, new_ckpt
-
-
-def _eval_only(kind, dataset, tmp_path, name, flags, ckpt, dropin):
-    ev = [f for f in flags]
-    ev += ["-eval_only_mode", "-load_experiment_name", ckpt]
-    log, _, _ = H.run_driver(kind, ev, str(tmp_path), name, dropin=dropin, cpu=not dropin)
-    return log
-
-
-@needs_ref
-@pytest.mark.gpu
-@pytest.mark.parametrize("model_type,l1", [("transe", True), ("transh", False), ("transr", False)])
-def test_kg_driver_unchanged(dataset, tmp_path, model_type, l1):
-    flags = _flags(dataset, "-model_type", model_type, "-kg_test_files", "valid.dat", "-training_steps", "300",
-                   "-eval_interval_steps", "150") + (["-L1_flag"] if l1 else [])
-    ref, new, ref_ckpt, new_ckpt = _both("kg", dataset, tmp_path, model_type, flags)
-    keys = ("train_loss", "kg", "kg_head", "kg_tail")
-    if model_type == "transr":
-        # The drivers add normLoss = sum max(|row|^2 - 1, 0) over rows that START on the unit sphere (|row|^2 = 1 +- 1 ulp),
-        # so which rows get its 2 x gradient on step 0 depends on the reduction order of torch.sum on the device the driver's
-        # own regulariser code runs on (CPU vs GPU) -- a property of the reference, outside the scoring kernels
-        # (profiles/diag_transr_step.py: scores agree to 2e-7, the regulariser's gradient differs).  TransR's unnormalised
-        # d x d matrices amplify that seed; TransE / TransH stay within the tight bounds.
-        _compare_logs(ref, new, keys, loss_rel=3e-2, frac_abs=0.01, rank_rel=0.05)
-    else:
-        _compare_logs(ref, new, keys)
-    assert ref["kg"][-1][1] < ref["kg"][0][1]          # training moved the mean rank
-    # checkpoints interchange: each side evaluates the other's best checkpoint (trainer.py:109-142)
-    a = _eval_only("kg", dataset, tmp_path, model_type + "_refckpt_on_b200", flags, ref_ckpt, dropin=True)
-    b = _eval_only("kg", dataset, tmp_path, model_type + "_b200ckpt_on_ref", flags, new_ckpt, dropin=False)
-    _compare_logs({"kg": [ref["kg"][-1]]}, {"kg": [a["kg"][-1]]}, ("kg",), frac_abs=0.005, rank_rel=0.002)
-    _compare_logs({"kg": [new["kg"][-1]]}, {"kg": [b["kg"][-1]]}, ("kg",), frac_abs=0.005, rank_rel=0.002)
-
-
-@needs_ref
-@pytest.mark.gpu
-@pytest.mark.parametrize("gumbel", [False, True])
-def test_rec_driver_unchanged(dataset, tmp_path, gumbel):
-    name = "transup_gumbel" if gumbel else "transup_soft"
-    flags = _flags(dataset, "-model_type", "transup", "-rec_test_files", "valid.dat", "-num_preferences", "6",
-                   "-training_steps", "300", "-eval_interval_steps", "150") + (["-use_st_gumbel"] if gumbel else [])
-    ref, new, ref_ckpt, new_ckpt = _both("rec", dataset, tmp_path, name, flags)
-    if gumbel:
-        # the Gumbel noise comes from different generators (torch CPU mt19937 vs in-kernel Philox), in training
-        # and in evaluate (transUP.py:161 draws it even under model.eval()): statistical agreement only
-        _compare_logs(ref, new, ("train_loss", "rec"), loss_rel=0.05, frac_abs=0.06)
-    else:
-        # item_recommendation.py:177-180 adds normLoss over user / item / preference rows that start exactly on the unit
-        # sphere: which of them get its 2 x gradient on the first steps depends on the reduction order of the driver's own
-        # torch.sum on CPU vs GPU (see the TransR note in test_kg_driver_unchanged); with Adagrad's first steps being
-        # +-lr per element that seed is visible in the logged loss.  KTUP's rec branch has no such term and is held to
-        # the tight bounds (test_joint_driver_unchanged); here the exact check is the checkpoint interchange below.
-        _compare_logs(ref, new, ("train_loss", "rec"), loss_rel=0.05, frac_abs=0.01)
-        a = _eval_only("rec", dataset, tmp_path, name + "_refckpt_on_b200", flags, ref_ckpt, dropin=True)
-        _compare_logs({"rec": [ref["rec"][-1]]}, {"rec": [a["rec"][-1]]}, ("rec",), frac_abs=0.005)
-
-
-@needs_ref
-@pytest.mark.gpu
-def test_joint_driver_unchanged(dataset, tmp_path):
-    flags = _flags(dataset, "-model_type", "jtransup", "-rec_test_files", "valid.dat", "-kg_test_files", "valid.dat",
-                   "-joint_ratio", "0.5", "-training_steps", "300", "-eval_interval_steps", "150")
-    ref, new, ref_ckpt, new_ckpt = _both("joint", dataset, tmp_path, "jtransup", flags)
-    _compare_logs(ref, new, ("joint_loss", "rec", "kg"))
-    b = _eval_only("joint", dataset, tmp_path, "jtransup_b200ckpt_on_ref", flags, new_ckpt, dropin=False)
-    _compare_logs({"rec": [new["rec"][-1]], "kg": [new["kg"][-1]]}, {"rec": [b["rec"][-1]], "kg": [b["kg"][-1]]},
-                  ("rec", "kg"), frac_abs=0.005, rank_rel=0.002)
-
-
-@needs_ref
-@pytest.mark.gpu
-def test_bprmf_runs_beside_the_dropin(dataset, tmp_path):
-    """Models the drop-in does not replace (bprmf) still dispatch to the reference's own class."""
-    flags = _flags(dataset, "-model_type", "bprmf", "-rec_test_files", "valid.dat", "-training_steps", "60",
-                   "-eval_interval_steps", "30")
-    log, _, _ = H.run_driver("rec", flags, str(tmp_path), "bprmf_dropin", dropin=True)
-    assert len(log["rec"]) == 2
-
-
-@needs_ref
-def test_reference_trainer_checkpoints_and_warm_starts_the_cuda_modules(tmp_path, monkeypatch):
-    """The unchanged ModelTrainer (utils/trainer.py) around the drop-in modules, on the host (no scoring call is made):
-    `save` / `load` round-trip their state_dict (trainer.py:109-142) and `loadEmbedding` (144-205) -- the `-load_ckpt_file`
-    warm start of the joint model from a pre-trained TransH -- assigns rows through `.weight.data[mapped, :]` with the
-    entity remap, which requires the tables to be ordinary nn.Embedding weights under the reference's state_dict keys."""
-    import logging
-    import sys
-    import types
-    for p in reversed(H.make_ref.env_paths()):
-        if p not in sys.path:
-            sys.path.insert(0, p)
-    import gflags  # noqa: F401
-    monkeypatch.setenv("TORCH_FORCE_NO_WEIGHTS_ONLY_LOAD", "1")          # the trainer reloads numpy scalars with a bare torch.load
-    from jTransUP.utils.trainer import ModelTrainer
-    import kgrec_b200 as K
-    flags = types.SimpleNamespace(model_type="transh", optimizer_type="Adagrad", l2_lambda=0.0, learning_rate=0.05,
-                                  learning_rate_decay_when_no_progress=0.5, momentum=0.9, eval_interval_steps=10,
-                                  ckpt_path=str(tmp_path), experiment_name="pre", eval_only_mode=False, load_experiment_name="")
-    log = logging.getLogger("kgrec_test")
-    torch.manual_seed(3)
-    E, R, d = 40, 5, 16
-    pre = K.TransHModel(True, d, E, R)
-    tr = ModelTrainer(pre, log, 10, flags)
-    tr.step, tr.best_step, tr.best_dev_performance = 30, 20, np.float64(0.4)
-    tr.checkpoint()
-    ck = os.path.join(str(tmp_path), "pre.ckpt")
-    assert os.path.exists(ck)
-    # plain reload into a second instance through the trainer
-    other = K.TransHModel(True, d, E, R)
-    tr2 = ModelTrainer(other, log, 10, flags)
-    tr2.load(ck, cpu=True)
-    assert (tr2.step, tr2.best_step, float(tr2.best_dev_performance)) == (30, 20, 0.4)
-    for k, v in pre.state_dict().items():
-        assert torch.equal(v.cpu(), other.state_dict()[k].cpu()), k
-    # warm start of the joint model (-load_ckpt_file).  A pre-trained table with exactly one row less than the joint
-    # model's (E vs E + 1 with the padding row) takes the trainer's "cke" branch: rows copied in place, no remap.
-    U, I = 7, 9
-    i_map = {i: i for i in range(I)}
-    new_map = {i: ((i * 3) % E if i % 2 else -1, i) for i in range(I)}
-    names = ["ent_embeddings.weight", "rel_embeddings.weight", "norm_embeddings.weight"]
-    jflags = types.SimpleNamespace(**dict(vars(flags), model_type="jtransup", experiment_name="joint"))
-    joint = K.jTransUPModel(True, d, U, I, E, R, i_map, new_map, False, False)
-    before_user = joint.user_embeddings.weight.detach().clone()
-    ModelTrainer(joint, log, 10, jflags).loadEmbedding(ck, names, cpu=True, e_remap={e: (e * 7) % E for e in range(E)})
-    ent_pre = pre.ent_embeddings.weight.detach().cpu()
-    ent_new = joint.ent_embeddings.weight.detach().cpu()
-    assert ent_new.shape[0] == E + 1 and torch.equal(ent_new[:E], ent_pre)
-    assert not ent_new[E].any()                                       # the padding row stays zero (jTransUP.py:96-100)
-    assert torch.equal(joint.rel_embeddings.weight.detach().cpu(), pre.rel_embeddings.weight.detach().cpu())
-    assert torch.equal(joint.norm_embeddings.weight.detach().cpu(), pre.norm_embeddings.weight.detach().cpu())
-    assert torch.equal(joint.user_embeddings.weight.detach().cpu(), before_user.cpu())
-    # a joint vocabulary that is larger than the pre-trained one: rows go through e_remap (trainer.py:176-186)
-    E2 = E + 6
-    big = K.jTransUPModel(True, d, U, I, E2, R, i_map, new_map, False, False)
-    untouched = big.ent_embeddings.weight.detach().clone()
-    e_remap = {e: (e * 7) % E2 for e in range(E)}                     # old entity id -> joint index (injective: gcd(7, 46) = 1)
-    assert len(set(e_remap.values())) == E
-    ModelTrainer(big, log, 10, jflags).loadEmbedding(ck, names, cpu=True, e_remap=e_remap)
-    ent_big = big.ent_embeddings.weight.detach().cpu()
-    for e, m in e_remap.items():
-        assert torch.equal(ent_big[m], ent_pre[e])
-    rest = sorted(set(range(E2 + 1)) - set(e_remap.values()))
-    assert torch.equal(ent_big[rest], untouched.cpu()[rest])          # rows without a pre-trained counterpart keep their init
+        want = {k[len(name) + 1:]: v for k, v in g.items() if k.startswith(name + "/") and k != name + "/rand"}
+        sb = b.state_dict()
+        assert set(want) == set(sb), name
+        for k in want:
+            assert np.array_equal(want[k], sb[k].cpu().numpy()), (name, k)
+        assert np.array_equal(g[name + "/rand"], rb.numpy())

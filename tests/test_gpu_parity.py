@@ -1569,3 +1569,35 @@ def test_device_prefetcher_ring_reuse():
     assert [int(s) for s in sums] == want
     for a, b in zip(DevicePrefetcher(iter(host[:3]), "cuda"), host[:3]):     # a second pass reuses the ring
         assert torch.equal(a[0].cpu(), b[0]) and torch.equal(a[1].cpu(), b[1])
+
+
+def test_bench_dump_outputs_are_repeatable(tmp_path):
+    """`bench.py --dump-outputs DIR`: the last timed launch's losses, scores and a seeded sample of its gradient rows,
+    float32 / float64, under 64 MB, the same from run to run with the same arguments (the inputs are seeded)."""
+    import json
+    import os
+    import subprocess
+    import sys
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    nb = 2
+    runs = []
+    for i in range(2):
+        out = tmp_path / ("run%d" % i)
+        cmd = [sys.executable, os.path.join(root, "bench.py"), "--steps", "2", "--warmup", "1", "--batches-per-step", str(nb),
+               "--launches-per-step", "2", "--headline-only", "--no-eval", "--no-cpu-baseline", "--dump-outputs", str(out)]
+        r = subprocess.run(cmd, capture_output=True, text=True, timeout=600, cwd=str(tmp_path))
+        assert r.returncode == 0, r.stderr[-2000:]
+        assert json.loads(r.stdout.strip().splitlines()[-1])["steps"] == 2
+        runs.append({f[:-4]: np.load(str(out / f)) for f in sorted(os.listdir(str(out)))})
+    a, b = runs
+    assert set(a) == {"loss_per_batch", "pos_scores", "neg_scores", "ent_grad_slots", "ent_grad_rows", "ent_grad_values",
+                      "rel_grad_slots", "rel_grad_rows", "rel_grad_values"}
+    assert sum(x.nbytes for x in a.values()) <= 64 << 20
+    assert a["loss_per_batch"].shape == (nb,) and a["pos_scores"].shape == (nb * 1024,)
+    assert a["neg_scores"].shape == (nb * 1024 * 10,) and a["ent_grad_values"].shape[1] == 100
+    for k in a:
+        assert a[k].dtype in (np.float32, np.float64), k
+        if k.endswith(("_slots", "_rows")):
+            assert np.array_equal(a[k], b[k]), k
+        else:                                   # a reduction may add in another order from run to run
+            np.testing.assert_allclose(a[k], b[k], rtol=1e-5, atol=1e-6, err_msg=k)
