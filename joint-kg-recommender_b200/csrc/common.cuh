@@ -2,6 +2,7 @@
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
+#include <type_traits>
 #include "../../include/kgrec_b200.h"
 
 namespace kgrec {
@@ -24,6 +25,16 @@ void set_error(const char* fmt, ...);
   } while (0)
 int sm_count();
 float l2_keep_fraction(double table_bytes);   // share of a table's lines worth pinning in L2
+
+// Launch dispatch on runtime flags: with_bools(f, a, b) calls f(std::integral_constant<bool, a>{}, ...), so f can
+// name a kernel template with the flags as template arguments; f is instantiated once per combination.
+template <typename F>
+inline void with_bools(F&& f) { f(); }
+template <typename F, typename... Bs>
+inline void with_bools(F&& f, bool b, Bs... bs) {
+  auto bind = [&](auto c) { with_bools([&](auto... cs) { f(c, cs...); }, bs...); };
+  if (b) bind(std::true_type{}); else bind(std::false_type{});
+}
 
 // ---- warp reductions --------------------------------------------------------
 __device__ __forceinline__ float warp_sum(float v) {
@@ -123,14 +134,6 @@ __device__ __forceinline__ void bulk_g2s(void* dst, const void* src, uint32_t by
                    smem_u32(dst)),
                "l"(src), "r"(bytes), "r"(smem_u32(bar))
                : "memory");
-}
-
-// Generic-proxy reads of a shared-memory buffer must be ordered before the async proxy (TMA) overwrites it.
-__device__ __forceinline__ void fence_proxy_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
-__device__ __forceinline__ float4 lds_f4(uint32_t addr) {
-  float4 r;
-  asm volatile("ld.shared.v4.f32 {%0,%1,%2,%3}, [%4];" : "=f"(r.x), "=f"(r.y), "=f"(r.z), "=f"(r.w) : "r"(addr));
-  return r;
 }
 
 // ---- L2 cache policies ---------------------------------------------------------------------

@@ -103,7 +103,6 @@ struct EvalArgs {
   // outputs
   float* out; int64_t ld_out;               // FULL
   uint64_t* part_keys; int k;               // TOPK: [n_splits][nq][k]
-  int rotate;                               // tile-issue duty rotates over the warps (0: warp 0 issues; KGREC_EVAL_ROTATE=0, A/B)
   uint32_t* thr_glob;                       // TOPK, tiled kernels: [nq] score bits no top-K entry of the call can exceed (shared by the pieces)
   const int64_t* filter_ptr; const int32_t* filter_ids;
   const float* gold_scores; const int32_t* gold_ids; int32_t* counts;   // RANK
@@ -619,7 +618,7 @@ k_eval_tiled(const EvalArgs A, const int stages, const int64_t units_per_cta) {
   if (my_units <= 0) return;
 
   // unit g (0-based within this CTA) -> catalog tile (u_begin + g) % n_tiles -> stage g % stages
-  auto issue_tile = [&](int64_t g) {          // called by all lanes of warp 0
+  auto issue_tile = [&](int64_t g) {          // called by all lanes of the issuing warp
     const int s = static_cast<int>(g % stages);
     const int64_t row0 = ((u_begin + g) % n_tiles) * TN;
     const int rows = static_cast<int>(min(static_cast<int64_t>(TN), A.n_cat - row0));
@@ -746,7 +745,7 @@ k_eval_tiled(const EvalArgs A, const int stages, const int64_t units_per_cta) {
       since = 0;
     }
     const int s = static_cast<int>(g % stages);
-    if (wid == (A.rotate ? static_cast<int>(g % kTiledWarps) : 0) && g + prefetch < my_units) issue_tile(g + prefetch);   // the issue duty rotates: no warp is always the late one
+    if (wid == static_cast<int>(g % kTiledWarps) && g + prefetch < my_units) issue_tile(g + prefetch);   // the issue duty rotates: no warp is always the late one
     const float* tile = tiles + static_cast<size_t>(s) * TN * pitch;
     const int64_t row0 = ti * TN;
     const int rows = static_cast<int>(min(static_cast<int64_t>(TN), A.n_cat - row0));
@@ -1318,11 +1317,6 @@ struct EvalPlan {
   int64_t units_per_cta;
 };
 
-static int eval_rotate() {
-  static const int v = [] { const char* e = getenv("KGREC_EVAL_ROTATE"); return (e && e[0] == '0') ? 0 : 1; }();
-  return v;
-}
-
 static int eval_plan(const kgrec_tables* T, int model, int side, int mode, const float* cat, int64_t cat_ld,
                      int64_t nq, int64_t n_cat, int k, bool have_qvec, EvalArgs* A, EvalPlan* pl) {
   if (!T) { set_error("tables is NULL"); return KGREC_ERR_INVALID; }
@@ -1375,7 +1369,7 @@ static int eval_plan(const kgrec_tables* T, int model, int side, int mode, const
     pl->units_per_cta = (total_units + ctas - 1) / ctas;
     pl->grid = static_cast<int>((total_units + pl->units_per_cta - 1) / pl->units_per_cta);
     pl->n_splits = static_cast<int>((n_tiles_t + pl->units_per_cta - 1) / pl->units_per_cta + 1);
-    A->T = *T; A->rotate = eval_rotate(); A->side = side; A->nq = nq; A->cat = cat; A->cat_ld = cat_ld; A->n_cat = n_cat;
+    A->T = *T; A->side = side; A->nq = nq; A->cat = cat; A->cat_ld = cat_ld; A->n_cat = n_cat;
     A->n_splits = pl->n_splits; A->tn = tn_t; A->k = k;
     return KGREC_OK;
   }
@@ -1401,7 +1395,7 @@ static int eval_plan(const kgrec_tables* T, int model, int side, int mode, const
     pl->units_per_cta = (total_units + ctas - 1) / ctas;
     pl->grid = static_cast<int>((total_units + pl->units_per_cta - 1) / pl->units_per_cta);
     pl->n_splits = static_cast<int>((n_tiles_t + pl->units_per_cta - 1) / pl->units_per_cta + 1);
-    A->T = *T; A->rotate = eval_rotate(); A->side = side; A->nq = nq; A->cat = cat; A->cat_ld = cat_ld; A->n_cat = n_cat;
+    A->T = *T; A->side = side; A->nq = nq; A->cat = cat; A->cat_ld = cat_ld; A->n_cat = n_cat;
     A->n_splits = pl->n_splits; A->tn = 32; A->k = k;
     return KGREC_OK;
   }
@@ -1438,7 +1432,7 @@ static int eval_plan(const kgrec_tables* T, int model, int side, int mode, const
     pl->grid = static_cast<int>((total_units + pl->units_per_cta - 1) / pl->units_per_cta);
     // pieces of partial top-K lists per query tile: CTAs whose ranges touch one query tile
     pl->n_splits = static_cast<int>((n_tiles_t + pl->units_per_cta - 1) / pl->units_per_cta + 1);
-    A->T = *T; A->rotate = eval_rotate(); A->side = side; A->nq = nq; A->cat = cat; A->cat_ld = cat_ld; A->n_cat = n_cat;
+    A->T = *T; A->side = side; A->nq = nq; A->cat = cat; A->cat_ld = cat_ld; A->n_cat = n_cat;
     A->n_splits = pl->n_splits; A->tn = tn_t; A->k = k;
     return KGREC_OK;
   }
@@ -1455,7 +1449,7 @@ static int eval_plan(const kgrec_tables* T, int model, int side, int mode, const
   pl->n_splits = static_cast<int>(splits);
   pl->smem = eval_smem_layout(pl->kind, mode, d, cat_ld, T->n_pref, tn, k).total;
   if (pl->smem > 220 * 1024) { set_error("eval: shared-memory budget exceeded (%zu bytes)", pl->smem); return KGREC_ERR_UNSUPPORTED; }
-  A->T = *T; A->rotate = eval_rotate();
+  A->T = *T;
   A->side = side;
   A->nq = nq;
   A->cat = cat;
@@ -1581,8 +1575,7 @@ extern "C" int kgrec_eval_topk(const kgrec_tables* tables, int model, int side, 
   if (pl.tiled || pl.soft_aug) {
     // unused pieces = empty lists; and, room permitting, the per-query bound the pieces share (0xffffffff = none yet)
     int64_t fill = need;
-    static const bool share = [] { const char* e = getenv("KGREC_EVAL_SHARE"); return !(e && e[0] == '0'); }();
-    if (share && pl.n_splits > 1 && workspace_bytes >= need + 4 * nq) {
+    if (pl.n_splits > 1 && workspace_bytes >= need + 4 * nq) {
       A.thr_glob = reinterpret_cast<uint32_t*>(static_cast<unsigned char*>(workspace) + need);
       fill = need + 4 * nq;
     }

@@ -13,7 +13,6 @@
 //
 // Reference arithmetic: transE.py:51-63, transH.py:58-71 (+ utils/misc.py:18-19),
 // utils/loss.py:8-16, 29-31; CPU restatement: oracle/kg_oracle.py.
-#include <cstdlib>
 #include "train_dev.cuh"
 
 namespace kgrec {
@@ -410,8 +409,8 @@ k_group_step(const GroupArgs G, const float up0, float* __restrict__ pos_scores,
 //     group ahead and handed out by shuffles, so the request for row k+1 leaves as soon as row k's
 //     arithmetic starts (with per-negative id loads the row request waited a full L2 round trip:
 //     48 % of the stall samples).
-template <bool L1, bool DENSE, bool MARGIN, int MINB, bool PF, bool REG, bool BWD, bool FWD = false>
-__global__ void __launch_bounds__(kThreads, MINB)
+template <bool L1, bool DENSE, bool MARGIN, bool REG, bool BWD, bool FWD = false>
+__global__ void __launch_bounds__(kThreads, 4)
 k_group_step_e(const GroupArgs G, const float up0, const float* __restrict__ up_dev, float* __restrict__ pos_scores,
                float* __restrict__ neg_scores, float* __restrict__ group_loss, const kgrec_grads Gr,
                int64_t* __restrict__ slot_ent, int64_t* __restrict__ slot_rel, int32_t* status) {
@@ -479,7 +478,7 @@ k_group_step_e(const GroupArgs G, const float up0, const float* __restrict__ up_
       r = ldg_f4_hint(row(rel_b, ir), pol_keep);
       xa = ldg_f4_hint(row(ent_b, ida), pol_keep);
     }
-    if (PF && lane >= 2 && lane < K) {     // lane l holds the id of negative l: it pulls that row's lines towards the SM
+    if (lane >= 2 && lane < K) {     // lane l holds the id of negative l: it pulls that row's lines towards the SM
       const uint32_t pid = static_cast<uint32_t>(cv < 0 ? ~cv : cv);
       if (pid < n_ent) {
         const char* pr = reinterpret_cast<const char*>(T.ent) + static_cast<uint64_t>(pid) * ld4;
@@ -620,179 +619,6 @@ k_group_step_e(const GroupArgs G, const float up0, const float* __restrict__ up_
   if (bad && status) *status = 1;
 }
 
-// --- TransE, d <= 128: the step kernel with its gather STAGED THROUGH SHARED MEMORY BY TMA ----------------------
-// north_star: "128-bit vectorised coalesced HBM loads staged through TMA into shared memory".  Every row of a
-// group -- h, t, r and the K corrupted entities -- is fetched by ONE cp.async.bulk (400 B at d = 100) issued by the
-// lane that holds its id, into the warp's own ring of S stages; a stage carries an mbarrier armed with the group's
-// byte count, so the warp waits once per group and then reads its rows with conflict-free LDS.128 (lane = chunk).
-// The ring is warp-local (the same warp produces and consumes: no CTA barrier, no empty-slot barrier -- program
-// order plus a proxy fence orders the reads of a stage before the bulk copies that refill it), and it keeps
-// (S - 1) x (3 + K) x 400 B per warp in flight without holding a register: 125 KB per SM at 8 warps x 4 stages.
-// The arithmetic and the gradient stores are k_group_step_e's.  Whether this beats register loads + L1 prefetch
-// depends on where the table lives: profiles/r02_tma_gather_ab.json (L2-resident 100k entities vs 500k / 5M).
-template <bool L1, bool DENSE, bool MARGIN, int W>
-__global__ void __launch_bounds__(W * 32, 1)
-k_group_step_e_tma(const GroupArgs G, const float up0, float* __restrict__ pos_scores, float* __restrict__ neg_scores,
-                   float* __restrict__ group_loss, const kgrec_grads Gr, int64_t* __restrict__ slot_ent,
-                   int64_t* __restrict__ slot_rel, int32_t* status, const int S) {
-  extern __shared__ __align__(128) unsigned char smem_raw[];
-  const kgrec_tables& T = G.T;
-  const LossCfg& L = G.L;
-  const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
-  const int K = L.n_neg, n_rows = 3 + K;
-  const int n_pos = static_cast<int>(L.n_pos);
-  const uint32_t n_ent = static_cast<uint32_t>(T.n_ent);
-  const uint32_t ld4 = static_cast<uint32_t>(T.ld) * 4u, d4 = static_cast<uint32_t>(T.dim) * 4u;
-  const int bp = static_cast<int>(L.batch_pos < 0x7fffffff ? L.batch_pos : 0x7fffffff);
-  const uint64_t pol_stream = policy_evict_first();
-  const bool act = lane * 4 < T.dim;
-  // shared-memory map: [W][S] mbarriers | [W][S][32] int32 compact ids | [W][S][n_rows] rows of d4 bytes
-  uint64_t* bars = reinterpret_cast<uint64_t*>(smem_raw) + wid * S;
-  int32_t* ids_ring = reinterpret_cast<int32_t*>(smem_raw + static_cast<size_t>(W) * S * 8) + wid * S * 32;
-  const uint32_t stage_bytes = static_cast<uint32_t>(n_rows) * d4;
-  unsigned char* rows_base = smem_raw + ((static_cast<size_t>(W) * S * (8 + 128) + 127) & ~static_cast<size_t>(127)) +
-                             static_cast<size_t>(wid) * S * stage_bytes;
-  if (lane == 0)
-    for (int s = 0; s < S; ++s) mbar_init(bars + s, 1);
-  mbar_fence_init();
-  __syncwarp();
-  char* gent_b = reinterpret_cast<char*>(Gr.ent) + lane * 16;
-  char* grel_b = reinterpret_cast<char*>(Gr.rel) + lane * 16;
-  const float prm = L.param;
-  const int stride = gridDim.x * W;
-  const float4 z4 = make_float4(0.f, 0.f, 0.f, 0.f);
-  bool bad = false;
-  const void* pcol = lane == 0 ? G.ph : (lane == 1 ? G.pt : G.pr);
-
-  // producer half: ids of group jj -> ring slot, one bulk copy per row
-  auto issue = [&](int jj, int s) {
-    // lane 0..2: h, t, r of the positive; lane 3..3+K-1: corrupted entity of negative lane-3 (sign = head replaced)
-    int32_t v = 0;
-    if (lane < 3) {
-      const int64_t pv = load_idx(pcol, jj, G.is64);
-      const int64_t lim = lane == 2 ? T.n_rel : T.n_ent;
-      if (static_cast<uint64_t>(pv) >= static_cast<uint64_t>(lim)) bad = true; else v = static_cast<int32_t>(pv);
-    } else if (lane < n_rows) {
-      v = __ldg(G.corrupt + static_cast<uint32_t>(jj) * K + (lane - 3));
-      const uint32_t id = static_cast<uint32_t>(v < 0 ? ~v : v);
-      if (id >= n_ent) { bad = true; v = 0; }
-    }
-    ids_ring[s * 32 + lane] = v;
-    if (lane == 0) mbar_arrive_expect_tx(bars + s, stage_bytes);
-    __syncwarp();
-    if (lane < n_rows) {
-      const uint32_t id = lane < 3 ? static_cast<uint32_t>(v) : static_cast<uint32_t>(v < 0 ? ~v : v);
-      const char* src = reinterpret_cast<const char*>(lane == 2 ? T.rel : T.ent) + static_cast<uint64_t>(id) * ld4;
-      bulk_g2s(rows_base + static_cast<size_t>(s) * stage_bytes + static_cast<size_t>(lane) * d4, src, d4, bars + s);
-    }
-  };
-
-  int j = blockIdx.x * W + wid;
-  for (int s = 0, jj = j; s < S - 1 && jj < n_pos; ++s, jj += stride) issue(jj, s);
-  for (int it = 0; j < n_pos; j += stride, ++it) {
-    const int s = it % S;
-    {   // keep S - 1 groups in flight: refill the stage consumed in the previous iteration
-      const int jn = j + (S - 1) * stride;
-      if (jn < n_pos) {
-        fence_proxy_async_smem();
-        __syncwarp();
-        issue(jn, (it + S - 1) % S);
-      }
-    }
-    mbar_wait(bars + s, static_cast<uint32_t>(it / S) & 1u);
-    const int32_t myid = ids_ring[s * 32 + lane];
-    const uint32_t st_addr = smem_u32(rows_base + static_cast<size_t>(s) * stage_bytes) + lane * 16;
-    const uint32_t ih0 = static_cast<uint32_t>(__shfl_sync(FULL, myid, 0)), it0 = static_cast<uint32_t>(__shfl_sync(FULL, myid, 1)),
-                   ir0 = static_cast<uint32_t>(__shfl_sync(FULL, myid, 2));
-    if (slot_ent) {
-      const uint32_t s0 = static_cast<uint32_t>(j) * (2 + K);
-      if (lane < 2) slot_ent[s0 + lane] = myid;
-      if (lane == 2) slot_rel[j] = myid;
-      if (lane >= 3 && lane < n_rows) slot_ent[s0 + lane - 1] = myid < 0 ? ~myid : myid;
-    }
-    float4 h = z4, t = z4, r = z4;
-    if (act) { h = lds_f4(st_addr); t = lds_f4(st_addr + d4); r = lds_f4(st_addr + 2 * d4); }
-    float up = up0;
-    if (!MARGIN) {
-      const int b = j / bp;
-      up /= static_cast<float>(min(bp, n_pos - b * bp)) * static_cast<float>(K);
-    }
-    const float4 bh = make_float4(h.x + r.x, h.y + r.y, h.z + r.z, h.w + r.w);
-    const float4 bt = make_float4(t.x - r.x, t.y - r.y, t.z - r.z, t.w - r.w);
-    const float4 ep = make_float4(bh.x - t.x, bh.y - t.y, bh.z - t.z, bh.w - t.w);
-    const float sp = warp_sum(dist_term(ep.x, L1) + dist_term(ep.y, L1) + dist_term(ep.z, L1) + dist_term(ep.w, L1));
-    float lsum = 0.f, cpos = 0.f, mys = 0.f;
-    float4 accT = z4, accH = z4;
-    uint32_t goff = (static_cast<uint32_t>(j) * (2 + K) + 2) * d4;
-#pragma unroll 2
-    for (int k = 0; k < K; ++k) {
-      const int32_t c = __shfl_sync(FULL, myid, 3 + k);
-      const bool head = c < 0;
-      const uint32_t id = static_cast<uint32_t>(head ? ~c : c);
-      float4 x = z4;
-      if (act) x = lds_f4(st_addr + (3 + k) * d4);
-      const float4 B = head ? bt : bh;
-      const float4 e = make_float4(B.x - x.x, B.y - x.y, B.z - x.z, B.w - x.w);
-      const float sn = warp_sum(dist_term(e.x, L1) + dist_term(e.y, L1) + dist_term(e.z, L1) + dist_term(e.w, L1));
-      if (lane == k) mys = sn;
-      float coef;
-      if (MARGIN) {
-        const float tt = sp - sn + prm;
-        lsum += fmaxf(tt, 0.f);
-        coef = tt > 0.f ? up : 0.f;
-        cpos += tt > 0.f ? 1.f : 0.f;
-      } else {
-        const float xx = prm * (sp - sn);
-        lsum += fmaxf(-xx, 0.f) + log1pf(expf(-fabsf(xx)));
-        const float dp = -prm / (1.f + expf(xx));
-        cpos += dp;
-        coef = dp * up;
-      }
-      if (coef != 0.f) {
-        float4 gc;
-        if (L1) {
-          gc = make_float4(coef * ddist_term(e.x, 1), coef * ddist_term(e.y, 1), coef * ddist_term(e.z, 1), coef * ddist_term(e.w, 1));
-        } else {
-          const float c2 = 2.f * coef;
-          gc = make_float4(c2 * e.x, c2 * e.y, c2 * e.z, c2 * e.w);
-        }
-        if (head) { accH.x -= gc.x; accH.y -= gc.y; accH.z -= gc.z; accH.w -= gc.w; }
-        else { accT.x -= gc.x; accT.y -= gc.y; accT.z -= gc.z; accT.w -= gc.w; }
-        if (act) {
-          if (DENSE) red_add_f4(reinterpret_cast<float*>(gent_b + static_cast<uint64_t>(id) * d4), gc.x, gc.y, gc.z, gc.w);
-          else stg_f4_hint(reinterpret_cast<float4*>(gent_b + goff), gc.x, gc.y, gc.z, gc.w, pol_stream);
-        }
-      } else if (!DENSE) {
-        if (act) stg_f4_hint(reinterpret_cast<float4*>(gent_b + goff), 0.f, 0.f, 0.f, 0.f, pol_stream);
-      }
-      goff += d4;
-    }
-    const float cp = cpos * up;
-    const float4 eps = make_float4(cp * ddist_term(ep.x, L1), cp * ddist_term(ep.y, L1), cp * ddist_term(ep.z, L1), cp * ddist_term(ep.w, L1));
-    const float4 gh = make_float4(accT.x + eps.x, accT.y + eps.y, accT.z + eps.z, accT.w + eps.w);
-    const float4 gt = make_float4(accH.x - eps.x, accH.y - eps.y, accH.z - eps.z, accH.w - eps.w);
-    const float4 gr = make_float4(accT.x - accH.x + eps.x, accT.y - accH.y + eps.y, accT.z - accH.z + eps.z, accT.w - accH.w + eps.w);
-    if (lane == 0) {
-      pos_scores[j] = sp;
-      group_loss[j] = lsum;
-    }
-    if (lane < K) neg_scores[static_cast<uint32_t>(j) * K + lane] = mys;
-    if (act) {
-      if (DENSE) {
-        red_add_f4(reinterpret_cast<float*>(gent_b + static_cast<uint64_t>(ih0) * d4), gh.x, gh.y, gh.z, gh.w);
-        red_add_f4(reinterpret_cast<float*>(gent_b + static_cast<uint64_t>(it0) * d4), gt.x, gt.y, gt.z, gt.w);
-        red_add_f4(reinterpret_cast<float*>(grel_b + static_cast<uint64_t>(ir0) * d4), gr.x, gr.y, gr.z, gr.w);
-      } else {
-        const uint32_t g0 = static_cast<uint32_t>(j) * (2 + K) * d4;
-        stg_f4_hint(reinterpret_cast<float4*>(gent_b + g0), gh.x, gh.y, gh.z, gh.w, pol_stream);
-        stg_f4_hint(reinterpret_cast<float4*>(gent_b + g0 + d4), gt.x, gt.y, gt.z, gt.w, pol_stream);
-        stg_f4_hint(reinterpret_cast<float4*>(grel_b + static_cast<uint32_t>(j) * d4), gr.x, gr.y, gr.z, gr.w, pol_stream);
-      }
-    }
-  }
-  if (bad && status) *status = 1;
-}
-
 // --- TransH (and the KTUP KG branch), d <= 128: the same treatment ------------------------------
 // With proj(v) = v - (v.w) w the residual is e' = B - proj(x), B = proj(h) + r or proj(t) - r.  Writing
 // g = -eps' for the gradient arriving at proj(x), the group needs per negative only
@@ -802,8 +628,8 @@ k_group_step_e_tma(const GroupArgs G, const float up0, float* __restrict__ pos_s
 //   g_h = E_h - (E_h.w) w,  g_t = E_t - (E_t.w) w,  g_r = accT - accH + eps_p,
 //   g_w -= (E_h.w) h + (h.w) E_h + (E_t.w) t + (t.w) E_t.
 // The two reductions a negative needs after its residual (the score and g.w) share one shuffle tree.
-template <bool L1, bool DENSE, bool MARGIN, int MINB, bool PF, bool REG, bool BWD, bool FWD = false>
-__global__ void __launch_bounds__(kThreads, MINB)
+template <bool L1, bool DENSE, bool MARGIN, bool REG, bool BWD, bool FWD = false>
+__global__ void __launch_bounds__(kThreads, 3)
 k_group_step_h(const GroupArgs G, const float up0, const float* __restrict__ up_dev, float* __restrict__ pos_scores,
                float* __restrict__ neg_scores, float* __restrict__ group_loss, const kgrec_grads Gr,
                int64_t* __restrict__ slot_ent, int64_t* __restrict__ slot_rel, int32_t* status) {
@@ -873,7 +699,7 @@ k_group_step_h(const GroupArgs G, const float up0, const float* __restrict__ up_
       w = ldg_f4_hint(row(nrm_b, ir), pol_keep);
       xa = ldg_f4_hint(row(ent_b, ida), pol_keep);
     }
-    if (PF && lane >= 2 && lane < K) {     // lane l holds the id of negative l: it pulls that row's lines towards the SM
+    if (lane >= 2 && lane < K) {     // lane l holds the id of negative l: it pulls that row's lines towards the SM
       const uint32_t pid = static_cast<uint32_t>(cv < 0 ? ~cv : cv);
       if (pid < n_ent) {
         const char* pr = reinterpret_cast<const char*>(T.ent) + static_cast<uint64_t>(pid) * ld4;
@@ -1072,7 +898,7 @@ k_group_step_r(const GroupArgs G, const float up0, float* __restrict__ pos_score
   const int i_end = min(n_pos, (static_cast<int>(blockIdx.x) + 1) * chunk);
 
   for (int i = blockIdx.x * chunk + wid; i < i_end; i += kWarpsPerCta) {
-    const int j = order ? __ldg(order + i) : i;
+    const int j = __ldg(order + i);
     const int32_t cv = lane < K ? __ldg(G.corrupt + static_cast<int64_t>(j) * K + lane) : 0;
     const int64_t pv = lane < 3 ? load_idx(pcol, j, G.is64) : 0;
     const int64_t vh = __shfl_sync(FULL, pv, 0), vt = __shfl_sync(FULL, pv, 1), vr = __shfl_sync(FULL, pv, 2);
@@ -1399,7 +1225,7 @@ k_run_step_r(const GroupArgs G, const float up0, float* __restrict__ pos_scores,
     int j = -1;
     int64_t r = -1;
     if (lane < GC && i_from + lane < i_end) {
-      j = order ? __ldg(order + i_from + lane) : i_from + lane;
+      j = __ldg(order + i_from + lane);
       r = load_idx(G.pr, j, G.is64);
       if (static_cast<uint64_t>(r) >= static_cast<uint64_t>(T.n_rel)) { bad = true; r = 0; }
     }
@@ -1673,29 +1499,11 @@ k_rel_scatter(const void* pr, const int is64, const int n_pos, const int64_t n_r
 
 int make_plan(const kgrec_tables* T, int model, Plan* pl);
 
-// KGREC_GROUP_STEP is an A/B / test switch: read once, not on every call of the hot path.
-static const char* group_step_env() {
-  static const char* cached = [] { const char* e = getenv("KGREC_GROUP_STEP"); return e ? e : ""; }();
-  return cached[0] ? cached : nullptr;
-}
-
-// TMA-staged variant of the TransE step kernel: encoded as 16 * warps + stages, 0 = register-load kernel.
-// KGREC_GROUP_STEP=t<w><s> forces it (w: 8 -> 8 warps, c -> 12, g -> 16; s = stages 2..6), anything else the default.
-static int group_step_tma_mode(const kgrec_tables* T, int n_neg, int reg_flags) {
-  const char* env = group_step_env();
-  if (reg_flags) return 0;
-  if (env && env[0] == 't' && env[1] && env[2]) {
-    const int W = env[1] == '8' ? 8 : (env[1] == 'c' ? 12 : 16), S = env[2] - '0';
-    if (S < 2 || S > 6) return 0;
-    const size_t smem = static_cast<size_t>(W) * S * (136 + static_cast<size_t>(3 + n_neg) * T->dim * 4) + 128;
-    return smem <= 225 * 1024 ? 16 * W + S : 0;
-  }
-  return 0;
-}
-
+// Checks the arguments of a corrupt-format call and builds its kernel arguments.  small32: 32-bit slot offsets
+// suffice and a group's scores fit in the lanes of a warp, as the d <= 128 step kernels need.
 static int group_check(const kgrec_tables* T, int model, Plan* pl, const void* ph, const void* pt, const void* pr,
                        int idx_bytes, int64_t n_pos, const int32_t* corrupt, int32_t n_neg, int64_t batch_pos,
-                       int loss_kind, bool allow_r = false) {
+                       int loss_kind, float margin_or_target, GroupArgs* G, bool* small32, bool allow_r = false) {
   int rc = make_plan(T, model, pl);
   if (rc) return rc;
   if (pl->fam != FAM_E && pl->fam != FAM_H && !(allow_r && pl->fam == FAM_R)) {
@@ -1708,6 +1516,10 @@ static int group_check(const kgrec_tables* T, int model, Plan* pl, const void* p
   if (loss_kind != KGREC_LOSS_MARGIN && loss_kind != KGREC_LOSS_BPR) { set_error("unknown loss %d", loss_kind); return KGREC_ERR_INVALID; }
   if (n_pos < 0 || n_pos > 0x7fffffff || n_neg < 1 || batch_pos < 1) { set_error("bad n_pos / n_neg / batch_pos"); return KGREC_ERR_INVALID; }
   if (T->n_ent > 0x7fffffffll) { set_error("corrupt format holds entity ids in 31 bits"); return KGREC_ERR_UNSUPPORTED; }
+  *G = GroupArgs{*T, ph, pt, pr, idx_bytes == 8, corrupt, LossCfg{loss_kind, margin_or_target, n_neg, n_pos, batch_pos},
+                 l2_keep_fraction(static_cast<double>(T->n_ent) * T->ld * sizeof(float))};
+  *small32 = n_neg <= 32 && static_cast<double>(n_pos) * (2 + n_neg) * T->dim * 4 < 4.0e9 &&
+             static_cast<double>(n_pos) * n_neg < 2.0e9;
   return KGREC_OK;
 }
 
@@ -1728,34 +1540,26 @@ extern "C" int kgrec_corrupt_loss_fwd(const kgrec_tables* tables, int model, con
                                       float* pos_scores, float* neg_scores, float* loss, void* workspace,
                                       int32_t* status, kgrec_stream_t stream) {
   Plan pl;
-  int rc = group_check(tables, model, &pl, ph, pt, pr, idx_bytes, n_pos, corrupt, n_neg, batch_pos, loss_kind);
+  GroupArgs G;
+  bool small32;
+  int rc = group_check(tables, model, &pl, ph, pt, pr, idx_bytes, n_pos, corrupt, n_neg, batch_pos, loss_kind,
+                       margin_or_target, &G, &small32);
   if (rc) return rc;
   if (!pos_scores || !neg_scores || !loss || !workspace) { set_error("output / workspace pointer is NULL"); return KGREC_ERR_INVALID; }
   if (n_pos == 0) return KGREC_OK;
-  const GroupArgs G{*tables, ph, pt, pr, idx_bytes == 8, corrupt, LossCfg{loss_kind, margin_or_target, n_neg, n_pos, batch_pos},
-                    l2_keep_fraction(static_cast<double>(tables->n_ent) * tables->ld * sizeof(float))};
   float* group_loss = static_cast<float*>(workspace);
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  const char* env = group_step_env();
-  const bool small32 = n_neg <= 32 && static_cast<double>(n_pos) * (2 + n_neg) * tables->dim * 4 < 4.0e9 &&
-                       static_cast<double>(n_pos) * n_neg < 2.0e9;
-  if (pl.fam == FAM_E && pl.nch == 1 && small32 && !(env && env[0] == '0')) {
+  if (pl.fam == FAM_E && pl.nch == 1 && small32) {
     // the TransE step kernel in forward-only mode (TransH: k_group_fwd measured faster, 1.06 vs 1.09 ms fwd+bwd)
-    const kgrec_grads nog{};
-#define CALL_F(KERN, MINBV, L1V, MV) KERN<L1V, false, MV, MINBV, true, false, false, true><<<grid_for(n_pos), kThreads, 0, st>>>(G, 1.f, nullptr, pos_scores, neg_scores, group_loss, nog, nullptr, nullptr, status)
-#define CALL_F4(KERN, MINBV)                                                                                        \
-  {                                                                                                                 \
-    const bool mg = loss_kind == KGREC_LOSS_MARGIN;                                                                 \
-    if (tables->l1) { if (mg) CALL_F(KERN, MINBV, true, true); else CALL_F(KERN, MINBV, true, false); }             \
-    else { if (mg) CALL_F(KERN, MINBV, false, true); else CALL_F(KERN, MINBV, false, false); }                      \
-  }
-    CALL_F4(k_group_step_e, 4)
-#undef CALL_F4
-#undef CALL_F
+    with_bools([&](auto l1, auto mg) {
+      k_group_step_e<l1, false, mg, false, false, true><<<grid_for(n_pos), kThreads, 0, st>>>(
+          G, 1.f, nullptr, pos_scores, neg_scores, group_loss, kgrec_grads{}, nullptr, nullptr, status);
+    }, tables->l1 != 0, loss_kind == KGREC_LOSS_MARGIN);
   } else {
-#define CALL(FAMV, NCHV)                                                                                                  \
-  if (tables->l1) k_group_fwd<FAMV, NCHV, true><<<grid_for(n_pos), kThreads, 0, st>>>(G, pos_scores, neg_scores, group_loss, status); \
-  else k_group_fwd<FAMV, NCHV, false><<<grid_for(n_pos), kThreads, 0, st>>>(G, pos_scores, neg_scores, group_loss, status);
+#define CALL(FAMV, NCHV)                                                                                             \
+  with_bools([&](auto l1) {                                                                                          \
+    k_group_fwd<FAMV, NCHV, l1><<<grid_for(n_pos), kThreads, 0, st>>>(G, pos_scores, neg_scores, group_loss, status); \
+  }, tables->l1 != 0);
   KGREC_GROUP_DISPATCH(CALL)
 #undef CALL
   }
@@ -1773,7 +1577,10 @@ extern "C" int kgrec_corrupt_loss_bwd(const kgrec_tables* tables, int model, con
                                       const float* grad_loss_dev, const kgrec_grads* grads, int64_t* slot_ent_ids,
                                       int64_t* slot_rel_ids, kgrec_stream_t stream) {
   Plan pl;
-  int rc = group_check(tables, model, &pl, ph, pt, pr, idx_bytes, n_pos, corrupt, n_neg, batch_pos, loss_kind);
+  GroupArgs G;
+  bool small32;
+  int rc = group_check(tables, model, &pl, ph, pt, pr, idx_bytes, n_pos, corrupt, n_neg, batch_pos, loss_kind,
+                       margin_or_target, &G, &small32);
   if (rc) return rc;
   if (!pos_scores || !neg_scores) { set_error("saved scores are NULL"); return KGREC_ERR_INVALID; }
   if ((slot_ent_ids == nullptr) != (slot_rel_ids == nullptr)) { set_error("slot_ent_ids and slot_rel_ids go together"); return KGREC_ERR_INVALID; }
@@ -1782,32 +1589,21 @@ extern "C" int kgrec_corrupt_loss_bwd(const kgrec_tables* tables, int model, con
     return KGREC_ERR_INVALID;
   }
   if (n_pos == 0) return KGREC_OK;
-  const GroupArgs G{*tables, ph, pt, pr, idx_bytes == 8, corrupt, LossCfg{loss_kind, margin_or_target, n_neg, n_pos, batch_pos},
-                    l2_keep_fraction(static_cast<double>(tables->n_ent) * tables->ld * sizeof(float))};
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  const char* env = group_step_env();
-  const bool small32 = n_neg <= 32 && static_cast<double>(n_pos) * (2 + n_neg) * tables->dim * 4 < 4.0e9 &&
-                       static_cast<double>(n_pos) * n_neg < 2.0e9;
-  if ((pl.fam == FAM_E || pl.fam == FAM_H) && pl.nch == 1 && small32 && !(env && env[0] == '0')) {
+  if (pl.nch == 1 && small32) {
     // the step kernels in backward mode (coefficients from the saved scores, upstream per batch)
     float* ps = const_cast<float*>(pos_scores);
     float* ns = const_cast<float*>(neg_scores);
-#define CALL_B(KERN, MINBV, L1V, DV, MV) KERN<L1V, DV, MV, MINBV, true, false, true><<<grid_for(n_pos), kThreads, 0, st>>>(G, grad_loss, grad_loss_dev, ps, ns, nullptr, *grads, slot_ent_ids, slot_rel_ids, nullptr)
-#define CALL_B8(KERN, MINBV)                                                                                                   \
-  {                                                                                                                            \
-    const bool dn = grads->mode == 1, mg = loss_kind == KGREC_LOSS_MARGIN;                                                     \
-    if (tables->l1) { if (dn) { if (mg) CALL_B(KERN, MINBV, true, true, true); else CALL_B(KERN, MINBV, true, true, false); }  \
-                      else { if (mg) CALL_B(KERN, MINBV, true, false, true); else CALL_B(KERN, MINBV, true, false, false); } } \
-    else { if (dn) { if (mg) CALL_B(KERN, MINBV, false, true, true); else CALL_B(KERN, MINBV, false, true, false); }           \
-           else { if (mg) CALL_B(KERN, MINBV, false, false, true); else CALL_B(KERN, MINBV, false, false, false); } }          \
-  }
-    if (pl.fam == FAM_E) CALL_B8(k_group_step_e, 4) else CALL_B8(k_group_step_h, 3)
-#undef CALL_B8
-#undef CALL_B
+    with_bools([&](auto l1, auto dn, auto mg) {
+      auto kern = pl.fam == FAM_E ? k_group_step_e<l1, dn, mg, false, true> : k_group_step_h<l1, dn, mg, false, true>;
+      kern<<<grid_for(n_pos), kThreads, 0, st>>>(G, grad_loss, grad_loss_dev, ps, ns, nullptr, *grads, slot_ent_ids,
+                                                   slot_rel_ids, nullptr);
+    }, tables->l1 != 0, grads->mode == 1, loss_kind == KGREC_LOSS_MARGIN);
   } else {
-#define CALL(FAMV, NCHV)                                                                                                  \
-  if (tables->l1) k_group_bwd<FAMV, NCHV, true><<<grid_for(n_pos), kThreads, 0, st>>>(G, pos_scores, neg_scores, grad_loss, grad_loss_dev, *grads); \
-  else k_group_bwd<FAMV, NCHV, false><<<grid_for(n_pos), kThreads, 0, st>>>(G, pos_scores, neg_scores, grad_loss, grad_loss_dev, *grads);
+#define CALL(FAMV, NCHV)                                                                                               \
+  with_bools([&](auto l1) {                                                                                            \
+    k_group_bwd<FAMV, NCHV, l1><<<grid_for(n_pos), kThreads, 0, st>>>(G, pos_scores, neg_scores, grad_loss, grad_loss_dev, *grads); \
+  }, tables->l1 != 0);
   KGREC_GROUP_DISPATCH(CALL)
 #undef CALL
     if (slot_ent_ids) {
@@ -1834,7 +1630,10 @@ extern "C" int kgrec_corrupt_loss_step(const kgrec_tables* tables, int model, co
                                        const kgrec_grads* grads, int64_t* slot_ent_ids, int64_t* slot_rel_ids,
                                        void* workspace, int32_t* status, kgrec_stream_t stream) {
   Plan pl;
-  int rc = group_check(tables, model, &pl, ph, pt, pr, idx_bytes, n_pos, corrupt, n_neg, batch_pos, loss_kind, true);
+  GroupArgs G;
+  bool small32;
+  int rc = group_check(tables, model, &pl, ph, pt, pr, idx_bytes, n_pos, corrupt, n_neg, batch_pos, loss_kind,
+                       margin_or_target, &G, &small32, true);
   if (rc) return rc;
   if (!pos_scores || !neg_scores || !loss || !workspace) { set_error("output / workspace pointer is NULL"); return KGREC_ERR_INVALID; }
   if (!grads || (grads->mode != 0 && grads->mode != 1) || !grads->ent || !grads->rel || (pl.fam == FAM_H && !grads->norm) ||
@@ -1847,29 +1646,20 @@ extern "C" int kgrec_corrupt_loss_step(const kgrec_tables* tables, int model, co
     if (reg_flags) { set_error("fused regularisers are built for TransE / TransH"); return KGREC_ERR_UNSUPPORTED; }
     if (pl.nch != 1 || n_neg > 14) { set_error("TransR step kernel: embedding_size <= 128 and at most 14 negatives per positive"); return KGREC_ERR_UNSUPPORTED; }
     if (n_pos == 0) return KGREC_OK;
-    const GroupArgs GA{*tables, ph, pt, pr, idx_bytes == 8, corrupt, LossCfg{loss_kind, margin_or_target, n_neg, n_pos, batch_pos}, 1.f};
     float* gl = static_cast<float*>(workspace);
     cudaStream_t s2 = static_cast<cudaStream_t>(stream);
     // workspace: [group_loss n_pos | order n_pos | cursor n_rel]
     int32_t* order = reinterpret_cast<int32_t*>(gl + n_pos);
     int32_t* cursor = order + n_pos;
-    {
-      const char* env = group_step_env();
-      if (env && env[0] == 'u') order = nullptr;                      // KGREC_GROUP_STEP=u: batch order (A/B)
-    }
-    if (order) {
-      KGREC_CUDA_OK(cudaMemsetAsync(cursor, 0, sizeof(int32_t) * tables->n_rel, s2));
-      const int gs = static_cast<int>((n_pos + 255) / 256 < sm_count() * 4 ? (n_pos + 255) / 256 : sm_count() * 4);
-      k_rel_hist<<<gs, 256, 0, s2>>>(pr, idx_bytes == 8, static_cast<int>(n_pos), tables->n_rel, cursor);
-      k_rel_scan<<<1, 1024, 0, s2>>>(cursor, tables->n_rel);
-      k_rel_scatter<<<gs, 256, 0, s2>>>(pr, idx_bytes == 8, static_cast<int>(n_pos), tables->n_rel, cursor, order);
-    }
+    KGREC_CUDA_OK(cudaMemsetAsync(cursor, 0, sizeof(int32_t) * tables->n_rel, s2));
+    const int gs = static_cast<int>((n_pos + 255) / 256 < sm_count() * 4 ? (n_pos + 255) / 256 : sm_count() * 4);
+    k_rel_hist<<<gs, 256, 0, s2>>>(pr, idx_bytes == 8, static_cast<int>(n_pos), tables->n_rel, cursor);
+    k_rel_scan<<<1, 1024, 0, s2>>>(cursor, tables->n_rel);
+    k_rel_scatter<<<gs, 256, 0, s2>>>(pr, idx_bytes == 8, static_cast<int>(n_pos), tables->n_rel, cursor, order);
     const bool mg = loss_kind == KGREC_LOSS_MARGIN;
-    const char* env_r = group_step_env();
     // short runs (fewer than ~4 groups per relation of the table): staging M_r per tile does not pay, the warp kernel stays
-    const bool long_runs = n_pos >= 4 * tables->n_rel || (env_r && env_r[0] == 'r');
-    if (tables->dim >= 32 && long_runs && !(env_r && (env_r[0] == 'w' || env_r[0] == 'u'))) {
-      // the CTA-level run kernel; KGREC_GROUP_STEP=w keeps the warp-per-group kernel (A/B), =u that kernel in batch order
+    if (tables->dim >= 32 && n_pos >= 4 * tables->n_rel) {
+      // the CTA-level run kernel
       const int d = tables->dim, NC = d / 4, pitch = run_pitch(d), qf = d / 32;
       auto smem_for = [&](int rb) { return (2 * static_cast<size_t>(d) + 2 * 64 * rb) * pitch * 4 + 3 * 64 * rb * 8 + 72 * 4; };
       const int rb = (NC <= 27 && smem_for(2) <= 220 * 1024) ? 2 : 1;
@@ -1880,7 +1670,7 @@ extern "C" int kgrec_corrupt_loss_step(const kgrec_tables* tables, int model, co
   {                                                                                                                      \
     auto kern = mg ? k_run_step_r<QAV, QBV, QFV, RBV, true> : k_run_step_r<QAV, QBV, QFV, RBV, false>;                   \
     KGREC_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));       \
-    kern<<<grid, kThreads, smem, s2>>>(GA, grad_loss, pos_scores, neg_scores, gl, *grads, slot_ent_ids, slot_rel_ids, status, order); \
+    kern<<<grid, kThreads, smem, s2>>>(G, grad_loss, pos_scores, neg_scores, gl, *grads, slot_ent_ids, slot_rel_ids, status, order); \
   }
       if (NC <= 16) { if (qf <= 1) CALL_RUN(1, 1, 1, 2) else CALL_RUN(1, 1, 2, 2) }
       else if (NC <= 27) { if (qf <= 2) CALL_RUN(1, 3, 2, 2) else CALL_RUN(1, 3, 3, 2) }
@@ -1895,7 +1685,7 @@ extern "C" int kgrec_corrupt_loss_step(const kgrec_tables* tables, int model, co
   {                                                                                                                  \
     auto kern = k_group_step_r<NVTV, MV>;                                                                            \
     KGREC_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));   \
-    kern<<<grid_r, kThreads, smem, s2>>>(GA, grad_loss, pos_scores, neg_scores, gl, *grads, slot_ent_ids, slot_rel_ids, status, order); \
+    kern<<<grid_r, kThreads, smem, s2>>>(G, grad_loss, pos_scores, neg_scores, gl, *grads, slot_ent_ids, slot_rel_ids, status, order); \
   }
     if (nvt == 4) { if (mg) CALL_R(4, true) else CALL_R(4, false) }
     else if (nvt == 12) { if (mg) CALL_R(12, true) else CALL_R(12, false) }
@@ -1904,78 +1694,29 @@ extern "C" int kgrec_corrupt_loss_step(const kgrec_tables* tables, int model, co
     }
     KGREC_CUDA_OK(cudaGetLastError());
     const int64_t nbt = (n_pos + batch_pos - 1) / batch_pos;
-    k_batch_loss<<<static_cast<unsigned>(nbt), 256, 0, s2>>>(gl, GA.L, loss);
+    k_batch_loss<<<static_cast<unsigned>(nbt), 256, 0, s2>>>(gl, G.L, loss);
     KGREC_CUDA_OK(cudaGetLastError());
     return KGREC_OK;
   }
   if (n_pos == 0) return KGREC_OK;
-  const GroupArgs G{*tables, ph, pt, pr, idx_bytes == 8, corrupt, LossCfg{loss_kind, margin_or_target, n_neg, n_pos, batch_pos},
-                    l2_keep_fraction(static_cast<double>(tables->n_ent) * tables->ld * sizeof(float))};
   float* group_loss = static_cast<float*>(workspace);
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   if (reg_flags != 0 && reg_flags != 1) { set_error("reg_flags must be 0 or 1"); return KGREC_ERR_INVALID; }
   if (reg_flags && loss_kind != KGREC_LOSS_MARGIN) { set_error("fused regularisers go with the margin loss (the KG drivers' loss)"); return KGREC_ERR_UNSUPPORTED; }
-  // KGREC_GROUP_STEP (A/B runs, tests): 0 = the general kernel for every shape; n = no row prefetch;
-  // 3 (TransE) / 2 (TransH) = fewer CTAs per SM, no prefetch
-  const char* env = group_step_env();
-  const bool small32 = n_neg <= 32 && static_cast<double>(n_pos) * (2 + n_neg) * tables->dim * 4 < 4.0e9 &&
-                       static_cast<double>(n_pos) * n_neg < 2.0e9;          // 32-bit slot offsets, scores kept in lanes
-  const int tma_mode = group_step_tma_mode(tables, n_neg, reg_flags);   // TMA-staged gather (A/B switch or the size rule)
-  if (pl.fam == FAM_E && pl.nch == 1 && small32 && tma_mode && n_neg <= 29 && tables->ld == tables->dim) {
-    const int W = tma_mode / 16, S = tma_mode % 16;
-    const size_t smem = ((static_cast<size_t>(W) * S * (8 + 128) + 127) & ~static_cast<size_t>(127)) +
-                        static_cast<size_t>(W) * S * (3 + n_neg) * tables->dim * 4;
-    int64_t ctas = (n_pos + W - 1) / W;
-    if (ctas > sm_count()) ctas = sm_count();
-#define CALL_T(L1V, DV, MV, WV)                                                                                         \
-  {                                                                                                                     \
-    auto kern = k_group_step_e_tma<L1V, DV, MV, WV>;                                                                    \
-    KGREC_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));      \
-    kern<<<static_cast<int>(ctas), WV * 32, smem, st>>>(G, grad_loss, pos_scores, neg_scores, group_loss, *grads, slot_ent_ids, slot_rel_ids, status, S); \
-  }
-#define CALL_TW(L1V, DV, MV) { if (W == 8) CALL_T(L1V, DV, MV, 8) else if (W == 12) CALL_T(L1V, DV, MV, 12) else CALL_T(L1V, DV, MV, 16) }
-    const bool dn = grads->mode == 1, mg = loss_kind == KGREC_LOSS_MARGIN;
-    if (tables->l1) { if (dn) { if (mg) CALL_TW(true, true, true) else CALL_TW(true, true, false) } else { if (mg) CALL_TW(true, false, true) else CALL_TW(true, false, false) } }
-    else { if (dn) { if (mg) CALL_TW(false, true, true) else CALL_TW(false, true, false) } else { if (mg) CALL_TW(false, false, true) else CALL_TW(false, false, false) } }
-#undef CALL_TW
-#undef CALL_T
-  } else if (pl.fam == FAM_E && pl.nch == 1 && small32 && !(env && env[0] == '0')) {
-#define CALL_E(L1V, DV, MV)                                                                                      \
-  {                                                                                                              \
-    if (env && env[0] == 'n')                                                                                    \
-      k_group_step_e<L1V, DV, MV, 4, false, false, false><<<grid_for(n_pos), kThreads, 0, st>>>(G, grad_loss, nullptr, pos_scores, neg_scores, group_loss, *grads, slot_ent_ids, slot_rel_ids, status); \
-    else if (env && env[0] == '3')                                                                               \
-      k_group_step_e<L1V, DV, MV, 3, false, false, false><<<grid_for(n_pos), kThreads, 0, st>>>(G, grad_loss, nullptr, pos_scores, neg_scores, group_loss, *grads, slot_ent_ids, slot_rel_ids, status); \
-    else if (MV && reg_flags)                                                                                    \
-      k_group_step_e<L1V, DV, true, 4, true, true, false><<<grid_for(n_pos), kThreads, 0, st>>>(G, grad_loss, nullptr, pos_scores, neg_scores, group_loss, *grads, slot_ent_ids, slot_rel_ids, status); \
-    else                                                                                                         \
-      k_group_step_e<L1V, DV, MV, 4, true, false, false><<<grid_for(n_pos), kThreads, 0, st>>>(G, grad_loss, nullptr, pos_scores, neg_scores, group_loss, *grads, slot_ent_ids, slot_rel_ids, status); \
-  }
-    const bool dn = grads->mode == 1, mg = loss_kind == KGREC_LOSS_MARGIN;
-    if (tables->l1) { if (dn) { if (mg) CALL_E(true, true, true) else CALL_E(true, true, false) } else { if (mg) CALL_E(true, false, true) else CALL_E(true, false, false) } }
-    else { if (dn) { if (mg) CALL_E(false, true, true) else CALL_E(false, true, false) } else { if (mg) CALL_E(false, false, true) else CALL_E(false, false, false) } }
-#undef CALL_E
-  } else if (pl.fam == FAM_H && pl.nch == 1 && small32 && !(env && env[0] == '0')) {
-#define CALL_H(L1V, DV, MV)                                                                                      \
-  {                                                                                                              \
-    if (env && env[0] == 'n')                                                                                    \
-      k_group_step_h<L1V, DV, MV, 3, false, false, false><<<grid_for(n_pos), kThreads, 0, st>>>(G, grad_loss, nullptr, pos_scores, neg_scores, group_loss, *grads, slot_ent_ids, slot_rel_ids, status); \
-    else if (env && env[0] == '2')                                                                               \
-      k_group_step_h<L1V, DV, MV, 2, false, false, false><<<grid_for(n_pos), kThreads, 0, st>>>(G, grad_loss, nullptr, pos_scores, neg_scores, group_loss, *grads, slot_ent_ids, slot_rel_ids, status); \
-    else if (MV && reg_flags)                                                                                    \
-      k_group_step_h<L1V, DV, true, 3, true, true, false><<<grid_for(n_pos), kThreads, 0, st>>>(G, grad_loss, nullptr, pos_scores, neg_scores, group_loss, *grads, slot_ent_ids, slot_rel_ids, status); \
-    else                                                                                                         \
-      k_group_step_h<L1V, DV, MV, 3, true, false, false><<<grid_for(n_pos), kThreads, 0, st>>>(G, grad_loss, nullptr, pos_scores, neg_scores, group_loss, *grads, slot_ent_ids, slot_rel_ids, status); \
-  }
-    const bool dn = grads->mode == 1, mg = loss_kind == KGREC_LOSS_MARGIN;
-    if (tables->l1) { if (dn) { if (mg) CALL_H(true, true, true) else CALL_H(true, true, false) } else { if (mg) CALL_H(true, false, true) else CALL_H(true, false, false) } }
-    else { if (dn) { if (mg) CALL_H(false, true, true) else CALL_H(false, true, false) } else { if (mg) CALL_H(false, false, true) else CALL_H(false, false, false) } }
-#undef CALL_H
+  if (pl.nch == 1 && small32) {
+    with_bools([&](auto l1, auto dn, auto mg) {
+      const bool reg = mg && reg_flags;
+      auto kern = pl.fam == FAM_E ? (reg ? k_group_step_e<l1, dn, true, true, false> : k_group_step_e<l1, dn, mg, false, false>)
+                                  : (reg ? k_group_step_h<l1, dn, true, true, false> : k_group_step_h<l1, dn, mg, false, false>);
+      kern<<<grid_for(n_pos), kThreads, 0, st>>>(G, grad_loss, nullptr, pos_scores, neg_scores, group_loss, *grads,
+                                                   slot_ent_ids, slot_rel_ids, status);
+    }, tables->l1 != 0, grads->mode == 1, loss_kind == KGREC_LOSS_MARGIN);
   } else {
     if (reg_flags) { set_error("fused regularisers are built for the d <= 128 margin-loss step kernels only"); return KGREC_ERR_UNSUPPORTED; }
-#define CALL(FAMV, NCHV)                                                                                        \
-  if (tables->l1) k_group_step<FAMV, NCHV, true><<<grid_for(n_pos), kThreads, 0, st>>>(G, grad_loss, pos_scores, neg_scores, group_loss, *grads, status); \
-  else k_group_step<FAMV, NCHV, false><<<grid_for(n_pos), kThreads, 0, st>>>(G, grad_loss, pos_scores, neg_scores, group_loss, *grads, status);
+#define CALL(FAMV, NCHV)                                                                                                \
+  with_bools([&](auto l1) {                                                                                             \
+    k_group_step<FAMV, NCHV, l1><<<grid_for(n_pos), kThreads, 0, st>>>(G, grad_loss, pos_scores, neg_scores, group_loss, *grads, status); \
+  }, tables->l1 != 0);
   KGREC_GROUP_DISPATCH(CALL)
 #undef CALL
     if (slot_ent_ids) {

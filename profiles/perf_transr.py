@@ -14,7 +14,6 @@ def t(fn, reps=5):
     for _ in range(reps): fn()
     b.record(); torch.cuda.synchronize()
     return a.elapsed_time(b) / reps
-print("KGREC_GROUP_STEP =", os.environ.get("KGREC_GROUP_STEP", "(default: relation order)"))
 for nb, n_rel in ((32, 500), (32, 20), (1, 500), (1, 20)):
     ix = [x.to(dev) for x in bench.make_indices(torch, gen, nb)]
     pos, corrupt = (ix[0], ix[1], ix[2] % n_rel), ix[3]

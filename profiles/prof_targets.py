@@ -1,6 +1,6 @@
 """One small workload per kernel, for `ncu -k regex:<kernel>` captures (round 2).
     python profiles/prof_targets.py <target> [reps]
-targets: transr_step step_e100k step_e500k step_e5m step_tma5m eval_d128 eval_h_d128 opt transr_eval tup_step gumbel_eval soft_eval_d128"""
+targets: transr_step step_e100k step_e500k step_e5m eval_d128 eval_h_d128 opt transr_eval tup_step gumbel_eval soft_eval_d128"""
 import os, sys
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path[:0] = [ROOT, os.path.join(ROOT, "joint-kg-recommender_b200")]
@@ -24,7 +24,7 @@ def kg_ids(E, R=500, kn=KN):
 
 
 if target.startswith("step_"):
-    E = {"step_e100k": 100_000, "step_e500k": 500_000, "step_e5m": 5_000_000, "step_tma5m": 5_000_000}[target]
+    E = {"step_e100k": 100_000, "step_e500k": 500_000, "step_e5m": 5_000_000}[target]
     with device_init(dev):
         m = K.TransEModel(False, D, E, 500)
     m.grad_mode = "sparse"

@@ -14,7 +14,6 @@ cap() {   # name, kernel regex, target, skip
 cap r02_step_e100k k_group_step_e step_e100k 2
 cap r02_step_e500k k_group_step_e step_e500k 2 keep
 cap r02_step_e5m   k_group_step_e step_e5m 2
-KGREC_GROUP_STEP=tg2 cap r02_step_tma5m k_group_step_e_tma step_tma5m 2
 cap r02_eval_d128 k_eval_tiled eval_d128 1 keep
 cap r02_rows_update k_rows_update opt 2
 cap r02_rows_sqnorm k_rows_sqnorm opt 2
